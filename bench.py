@@ -2,7 +2,9 @@
 """Benchmark of the hot path: SD1.5 LoRA (rank 8, every attn1/attn2 Linear) training step, 512x512 (64x64 latents),
 batch 4 per GPU, bf16 kernels / fp32 master weights -- BASELINE.json `configs[1]`, metric "LoRA-train images/sec".
 
-  python bench.py [--gpus N] [--steps K] [--warmup W]            product arm (B200 kernels)
+  python bench.py [--gpus N] [--steps K] [--warmup W]            product arm (B200 kernels): K timed steps with inputs resident,
+                  [--dump-outputs DIR]                           then K timed steps fed from pinned host memory; DIR receives what
+                                                                 the last step left (see dump_outputs)
   python bench.py --impl reference [--gpus N] ...                CPU arm: the oracle restatement of the reference path
                                                                  (diffusers UNet semantics + hcpdiff LoRA operator + train_ac
                                                                  step order) on the host cores -- the reference itself cannot
@@ -296,6 +298,26 @@ def attn_tensor_pipe_pct():
     return out or None
 
 
+DUMP_MAX_PARAMS = 8 << 20        # float32 elements (32 MB): a larger parameter buffer is dumped as a fixed, seeded sample
+
+
+def dump_outputs(out_dir, step):
+    """What a caller of the training step holds after the last timed step: that step's loss (loss.npy, shape [1]) and the trainable
+    parameters AdamW left (params.npy: the flat fp32 parameter buffer, or DUMP_MAX_PARAMS elements of it at sorted indices drawn with
+    seed 0 when it is larger, e.g. the 860M parameters of --config 3).  Same arguments -> same inputs and step count, so the files of
+    two builds can be compared element for element.  They agree to a tolerance, not bitwise: the kernels' fp32 atomic accumulation
+    order varies, and two runs of one build on a B200 (1000 W) differed by 2e-5 (relative) in loss and 2e-3 relative L2 in the
+    parameters with --warmup 5 --steps 20."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    params = step.flat.data
+    if params.numel() > DUMP_MAX_PARAMS:
+        idx = torch.randint(0, params.numel(), (DUMP_MAX_PARAMS,), generator=torch.Generator().manual_seed(0)).sort().values
+        params = params[idx.to(params.device)]
+    np.save(os.path.join(out_dir, "loss.npy"), step.loss.detach().float().cpu().numpy())
+    np.save(os.path.join(out_dir, "params.npy"), params.detach().float().cpu().numpy())
+
+
 def run_product_arm(args, rank, world, local_rank):
     import torch.distributed as dist
     from hcp_diffusion_b200 import _lib
@@ -308,6 +330,8 @@ def run_product_arm(args, rank, world, local_rank):
     dev = torch.device("cuda", local_rank)
     _lib.check(_lib.lib().hcp_device_check(), "hcp_device_check")
     sustained, burst, hbm, peak_src = measured_peaks()
+    # the adapters draw W_down (kaiming-uniform) from the global generators on the device: seeded, so every run trains the same weights
+    torch.manual_seed(0)
 
     spec = U.SD15
     added = None
@@ -416,22 +440,16 @@ def run_product_arm(args, rank, world, local_rank):
     ms_resident = timed(resident_step, args.steps)
     clocks = sampler.stop()
     ms_e2e = timed(e2e_step, args.steps)
-    # sustained leg: at least 3 s of back-to-back steps (the short timed region above runs at boost clocks; a training job does not)
-    n_sus = max(args.steps, int(3200.0 / max(ms_resident / args.steps, 1e-3)) + 1)
-    sampler = ClockSampler(local_rank)
-    sampler.start()
-    ms_sus = timed(resident_step, n_sus)
-    clocks_sus = sampler.stop()
     assert all(l == l and l < 1e4 for l in losses), "loss diverged / NaN"
 
     if rank != 0:
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, step)
     imgs = world * B * args.steps
     value = imgs / (ms_resident * 1e-3)
     e2e_value = imgs / (ms_e2e * 1e-3)
-    sus_value = world * B * n_sus / (ms_sus * 1e-3)
     achieved = value / world * f_step * 1e-12
-    achieved_sus = sus_value / world * f_step * 1e-12
     # the denominator that matches the clocks this run saw: boost clocks for the whole timed region -> the burst peak
     boosted = bool(clocks.get("sm_mhz") and clocks.get("sm_max_mhz") and clocks["sm_mhz"] >= 0.9 * clocks["sm_max_mhz"])
     peak = burst if boosted else sustained
@@ -449,8 +467,6 @@ def run_product_arm(args, rank, world, local_rank):
                    "side_stream": os.environ.get("HCP_SIDE_STREAM", "1") != "0", "pdl": os.environ.get("HCP_PDL", "1") != "0"},
         "clocks": clocks,
         "e2e": {"value": e2e_value, "unit": "images/s", "ms_per_step": ms_e2e / args.steps, "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": 4},
-        "sustained": {"value": sus_value, "unit": "images/s", "steps": n_sus, "seconds": ms_sus * 1e-3, "ms_per_step": ms_sus / n_sus,
-                      "clocks": clocks_sus, "achieved_tflops": achieved_sus, "frac_of_sustained_peak": achieved_sus / sustained},
         "gpu_launches": launches_per_step * args.steps,
         "roofline": {"bound": "tensor", "achieved": achieved, "peak": peak, "unit": "TFLOP/s", "frac": achieved / peak,
                      "frac_vs_burst": achieved / burst, "frac_vs_sustained": achieved / sustained,
@@ -475,10 +491,16 @@ def main():
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="hcpb200", choices=["hcpb200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's loss and the trained parameters to DIR/<name>.npy (float32)")
     ap.add_argument("--config", type=int, default=2, choices=[2, 3, 4],
                     help="BASELINE.json config: 2 = SD1.5 LoRA r8 bs 4/GPU (the headline, default); 3 = SD1.5 full fine-tune bs 16/GPU; "
                          "4 = SDXL-base LoRA r16 attn + Conv2d bs 2/GPU, 1024x1024")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes what the product arm computed; the reference arm has no such output")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

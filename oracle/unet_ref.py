@@ -16,9 +16,8 @@ keys are the diffusers parameter names.  Structure follows the reference's modul
 
 LoRA semantics follow the reference operator exactly (``hcpdiff/models/lora_base_patch.py:21-35,61-74`` and
 ``hcpdiff/models/lora_layers_patch.py:44-57``): for every patched Linear, ``W' = W_host + sum_blocks alpha_b *
-(W_up_b @ W_down_b)`` is MATERIALISED and ``y = x @ W'^T + b``.  ``tests/test_oracle_reference_lora.py`` checks this
-against the real reference classes imported from ``/root/reference`` (when present) and against the committed golden
-vectors generated from them (``tests/golden/make_golden.py``).
+(W_up_b @ W_down_b)`` is MATERIALISED and ``y = x @ W'^T + b``.  ``tests/test_oracle.py`` checks this against the
+committed golden vectors generated from the real reference classes (``tests/golden/make_golden.py``).
 
 PARITY PINNING: the LoRA operator is pinned to the reference's own code; the UNet data flow is **parity unpinned** by the
 reference (it ships no tests, no golden vectors and not the diffusers code) -- it is defended structurally only

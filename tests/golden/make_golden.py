@@ -9,6 +9,7 @@ Outputs (small, committed):
                           checkpoint key names (the operator the CUDA kernels sit behind)
   ref_lora_dapp_conv.pt   the same for the DreamArtist++ pair (DAPPLayer / DAPPPatchContainer: batch = [negative | positive]) and
                           for LoraLayer on Conv2d hosts (3x3 stride 1 / stride 2 and 1x1)
+  ref_lora_wrap_layer.pt  LoraLayer.wrap_layer on a biased Linear (rank 8, alpha 2.0): weights, input and the reference output
   ref_step.pt             the step either side of the UNet, from the REAL reference code: MinSNRLoss / SoftMinSNRLoss / KDiffMinSNRLoss /
                           EDMLoss (hcpdiff/loss/min_snr_loss.py), a ModelEMA trajectory (hcpdiff/utils/ema.py), DreamArtistPTContext
                           pre/post (hcpdiff/models/cfg_context.py), get_cfg_range (hcpdiff/utils/utils.py), and DAPPLayer on a 3x3
@@ -205,6 +206,26 @@ def make_dapp_conv():
     print("ref_lora_dapp_conv.pt:", fx["container_types"], len(fx["grads"]), "lora grads")
 
 
+def make_wrap_layer():
+    """LoraLayer.wrap_layer on a biased Linear (rank 8, alpha 2.0, random W_up): host weights, adapter weights, input and the
+    output of the REAL reference layer."""
+    plugin, base, layers = import_reference_lora()
+    torch.manual_seed(3)
+    holder = nn.Module()
+    holder.lin = nn.Linear(40, 24, bias=True)
+    blk = layers.LoraLayer.wrap_layer(0, holder.lin, rank=8, alpha=2.0, parent_block=holder, host_name="lin")
+    with torch.no_grad():
+        blk.layer.W_up.normal_(0, 0.1)
+    x = torch.randn(5, 40)
+    with torch.no_grad():
+        out = holder.lin(x)
+    fx = {"weight": holder.lin._host.weight.detach().clone(), "bias": holder.lin._host.bias.detach().clone(),
+          "W_down": blk.layer.W_down.detach().clone(), "W_up": blk.layer.W_up.detach().clone(), "alpha": float(blk.alpha),
+          "x": x, "out": out.clone()}
+    torch.save(fx, os.path.join(HERE, "ref_lora_wrap_layer.pt"))
+    print("ref_lora_wrap_layer.pt: alpha", fx["alpha"], "out", tuple(out.shape))
+
+
 def make_webui_keys():
     """Key maps of the REAL reference LoraConverter (hcpdiff/tools/lora_convert.py) for the SD1.5 attention + ff LoRA layers."""
     import_reference_lora()
@@ -360,5 +381,6 @@ if __name__ == "__main__":
     make_struct()
     make_lora()
     make_dapp_conv()
+    make_wrap_layer()
     make_step()
     make_webui_keys()

@@ -1,11 +1,9 @@
 """CPU tests of the oracle (oracle/unet_ref.py): structure against the reference's module dump, LoRA semantics against
-vectors produced by the REAL reference classes (tests/golden/ref_lora_linear.pt, tests/golden/make_golden.py) and -- when
-/root/reference is present -- against the live reference classes."""
+vectors produced by the REAL reference classes (tests/golden/ref_lora_linear.pt, ref_lora_wrap_layer.pt,
+tests/golden/make_golden.py)."""
 import json
 import os
-import sys
 
-import pytest
 import torch
 
 from oracle import unet_ref as U
@@ -85,22 +83,14 @@ def test_oracle_lora_matches_reference_golden(golden_dir):
     assert abs(float(fx["ckpt"]["attn1.to_q.___.alpha"]) - 0.25) < 1e-7 and abs(float(fx["second_block"]["alpha"]) - 0.25) < 1e-7
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/hcpdiff"), reason="reference tree only exists in the build container")
-def test_oracle_lora_matches_live_reference_classes():
-    sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
-    import make_golden
-    plugin, base, layers = make_golden.import_reference_lora()
-    torch.manual_seed(3)
-    holder = torch.nn.Module()
-    holder.lin = torch.nn.Linear(40, 24, bias=True)
-    blk = layers.LoraLayer.wrap_layer(0, holder.lin, rank=8, alpha=2.0, parent_block=holder, host_name="lin")
-    with torch.no_grad():
-        blk.layer.W_up.normal_(0, 0.1)
-    x = torch.randn(5, 40)
-    ref = holder.lin(x)
-    sd = {"lin.weight": holder.lin._host.weight.detach(), "lin.bias": holder.lin._host.bias.detach()}
-    lora = {"lin": [U.LoraEntry(blk.layer.W_down.detach(), blk.layer.W_up.detach(), float(blk.alpha))]}
-    torch.testing.assert_close(U._linear(sd, lora, "lin", x), ref, rtol=1e-5, atol=1e-6)
+def test_oracle_lora_matches_live_reference_classes(golden_dir):
+    """The reference's LoraLayer.wrap_layer on a biased Linear (rank 8, alpha 2.0 -> 0.25 after auto scale): its output, stored in
+    tests/golden/ref_lora_wrap_layer.pt by tests/golden/make_golden.py, vs the oracle's `_linear` on the same weights and input."""
+    fx = torch.load(os.path.join(golden_dir, "ref_lora_wrap_layer.pt"))
+    sd = {"lin.weight": fx["weight"], "lin.bias": fx["bias"]}
+    lora = {"lin": [U.LoraEntry(fx["W_down"], fx["W_up"], fx["alpha"])]}
+    assert fx["W_down"].shape == (8, 40) and fx["alpha"] == 0.25
+    torch.testing.assert_close(U._linear(sd, lora, "lin", fx["x"]), fx["out"], rtol=1e-5, atol=1e-6)
 
 
 def test_tiny_unet_forward_backward_runs_and_is_deterministic():
